@@ -11,6 +11,8 @@ the timed region once, and is also timed alone (`allgather_us`).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--chunk 32] [--microbatch 32]
     ablations: --gather-every-step  --no-sampler  --no-graph  --op-by-op
+    --dump-outputs DIR: after the timed steps, the memory they left as DIR/<name>.npy (seeded inputs: two builds compare
+    output for output)
 
 Prints ONE JSON line (rank 0).  `value` = frames/s with inputs resident in HBM; `e2e` = the same through the public
 API from pinned HOST frames (H2D inside the timed region, D2H of the memory prefix every step).
@@ -54,7 +56,25 @@ def parse():
     ap.add_argument("--no-sampler", action="store_true", help="no nvidia-smi clock sampling")
     ap.add_argument("--no-graph", action="store_true", help="launch the ViT layer stack eagerly (FVS_VIT_GRAPH=0)")
     ap.add_argument("--op-by-op", action="store_true", help="op-by-op consolidation instead of fvs_stream_step")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the memory the last timed step left (rank 0) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return args
+
+
+def dump_outputs(out_dir, memory, buffer_frames=64):
+    """Write `video_embedding_memory` = [current, long, Turing, frame buffer], what a caller of embed_video_streaming
+    reads, as float32 DIR/<name>.npy.  The frame buffer holds one 8x8 map per frame of the stream (285 MB in float32 for
+    the default run), so only `buffer_frames` of its frames are written, picked by a fixed seed and kept in stream order."""
+    import numpy as np
+    cur, lng, tur, buf = memory
+    rows = np.sort(np.random.default_rng(0).choice(buf.shape[0], size=min(buf.shape[0], buffer_frames), replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"memory_current": cur, "memory_long": lng, "memory_turing": tur, "memory_buffer_sample": buf[rows.tolist()]}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+    return sorted(arrays)
 
 
 def peaks():
@@ -473,6 +493,8 @@ def run_b200(args):
     draws = stream_draws(n_total, 9000)
     step_resident, step_e2e = make_steps(draws)
     res = timed(step_resident, K, W, profile=not args.no_prof, prof_every=prof_every)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model.video_embedding_memory)
     res_e2e = timed(step_e2e, K, W, profile=False)
 
     # ---- the all-gather alone (once per query): microseconds per call, events around 20 back-to-back calls

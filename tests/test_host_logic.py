@@ -2,6 +2,7 @@
 calls — there is no GPU here), the Python mirror has the reference's signatures, the multi-GPU host logic works over
 gloo with world_size 2, and the product refuses to run without CUDA."""
 import inspect
+import json
 import os
 import re
 import subprocess
@@ -11,7 +12,6 @@ import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference/Flash-VStream-LLaVA"
 
 
 def header_functions():
@@ -31,7 +31,11 @@ def test_library_builds_loads_and_exports_every_declared_symbol():
         assert name in _lib.SIGNATURES, f"{name} has no ctypes signature"
     assert set(_lib.SIGNATURES) == set(declared)
     assert lib.fvs_version() >= 100
-    assert lib.fvs_launch_count() == 0
+    # a freshly loaded library has launched nothing (its own process: earlier tests of this one may have run kernels)
+    fresh = subprocess.run([sys.executable, "-c", "from flash_vstream_b200 import _lib; print(_lib.load().fvs_launch_count())"],
+                           cwd=ROOT, capture_output=True, text=True)
+    assert fresh.returncode == 0, fresh.stderr
+    assert fresh.stdout.strip() == "0"
 
 
 def test_sass_contains_blackwell_tensor_and_tma_instructions():
@@ -74,104 +78,118 @@ def test_unknown_sample_type_raises_like_reference():
         m.compress_spatial_features(torch.zeros(1, 60, 64), 4)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree only exists in the build container")
+def _seams():
+    """tests/golden/seams.json: what the original Flash-VStream modules define (tests/golden/make_golden_seams.py)"""
+    with open(os.path.join(ROOT, "tests", "golden", "seams.json")) as f:
+        return json.load(f)
+
+
+def _params(f):
+    """[name, repr(default) or None] of every parameter that is not keyword-only (the format of seams.json)"""
+    return [[p.name, None if p.default is p.empty else repr(p.default)]
+            for p in inspect.signature(f).parameters.values() if p.kind is not p.KEYWORD_ONLY]
+
+
+def _stand_in_modules(monkeypatch, names_by_module, classes=None):
+    """register, for the duration of a test, module objects under the original modules' import names that define the
+    names each original module defines (values are placeholders), so install() rebinds attributes on modules of the
+    original layout; returns {module name: module}"""
+    import types
+    mods = {}
+    for full, names in names_by_module.items():
+        parts = full.split(".")
+        for i in range(1, len(parts) + 1):
+            name = ".".join(parts[:i])
+            if name not in mods:
+                mod = types.ModuleType(name)
+                mod.__path__ = []
+                mods[name] = mod
+                monkeypatch.setitem(sys.modules, name, mod)
+                if i > 1:
+                    setattr(mods[".".join(parts[:i - 1])], parts[i - 1], mod)
+        for n in names:
+            setattr(mods[full], n, object())
+    for (full, cls_name), methods in (classes or {}).items():
+        setattr(mods[full], cls_name, type(cls_name, (), {m: object() for m in methods}))
+    return mods
+
+
 def test_mirror_signatures_match_reference():
-    sys.path.insert(0, REF)
-    from flash_vstream.model import compress_functions as rcf
-    from flash_vstream.model import vstream_arch as rarch
-    from flash_vstream.model.multimodal_encoder import clip_encoder as rclip
     from flash_vstream_b200 import clip_encoder as mclip
     from flash_vstream_b200 import compress_functions as mcf
     from flash_vstream_b200 import vstream_arch as march
-
-    def params(f, drop_kwonly=True):
-        ps = inspect.signature(f).parameters.values()
-        return [(p.name, p.default) for p in ps if not (drop_kwonly and p.kind is p.KEYWORD_ONLY)]
-
-    for name in ("weighted_kmeans_feature", "attention_feature", "drop_feature", "merge_feature", "kmeans_feature",
-                 "k_drop_feature", "k_merge_feature"):
-        assert params(getattr(mcf, name)) == params(getattr(rcf, name)), name
+    ref = _seams()["llava"]
+    for name, want in ref["compress_functions"].items():
+        assert _params(getattr(mcf, name)) == want, name
     for name in ("encode_images", "attention", "compress_spatial_features"):
-        assert params(getattr(march.VStreamMetaForCausalLM, name)) == params(getattr(rarch.VStreamMetaForCausalLM, name)), name
+        assert _params(getattr(march.VStreamMetaForCausalLM, name)) == ref["VStreamMetaForCausalLM"][name], name
     for name in ("compress_temporal_features", "embed_video_streaming"):   # ours add an optional trailing `draws=None`
-        mine = params(getattr(march.VStreamMetaForCausalLM, name))
-        assert mine[:-1] == params(getattr(rarch.VStreamMetaForCausalLM, name)) and mine[-1] == ("draws", None), name
-    assert params(mclip.CLIPVisionTower.__init__) == params(rclip.CLIPVisionTower.__init__)
-    assert params(mclip.CLIPVisionTower.forward) == params(rclip.CLIPVisionTower.forward)
-    ntm_ref = rarch.NeuralTuringMachine(64, 32).state_dict()
+        mine = _params(getattr(march.VStreamMetaForCausalLM, name))
+        assert mine[:-1] == ref["VStreamMetaForCausalLM"][name] and mine[-1] == ["draws", "None"], name
+    assert _params(mclip.CLIPVisionTower.__init__) == ref["CLIPVisionTower"]["__init__"]
+    assert _params(mclip.CLIPVisionTower.forward) == ref["CLIPVisionTower"]["forward"]
     ntm_mine = march.NeuralTuringMachine(64, 32).state_dict()
-    assert {k: v.shape for k, v in ntm_ref.items()} == {k: v.shape for k, v in ntm_mine.items()}
+    assert {k: list(v.shape) for k, v in ntm_mine.items()} == ref["ntm_64_32_state_dict"]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree only exists in the build container")
-def test_install_rebinds_reference_seam():
-    sys.path.insert(0, REF)
+def test_install_rebinds_reference_seam(monkeypatch):
     import flash_vstream_b200
-    from flash_vstream.model import compress_functions as rcf
-    from flash_vstream.model import vstream_arch as rarch
-    keep = (rcf.weighted_kmeans_feature, rarch.VStreamMetaForCausalLM.embed_video_streaming)
+    from flash_vstream_b200 import clip_encoder as mclip
+    from flash_vstream_b200 import compress_functions as mcf
+    from flash_vstream_b200 import multimodal_projector as mproj
+    from flash_vstream_b200 import vstream_arch as march
+    ref = _seams()["llava"]
+    arch = "flash_vstream.model.vstream_arch"
+    mods = _stand_in_modules(monkeypatch, ref["modules"],
+                             {(arch, "VStreamMetaForCausalLM"): ref["VStreamMetaForCausalLM_methods"]})
+    rcf, rarch = mods["flash_vstream.model.compress_functions"], mods[arch]
+    Ref = rarch.VStreamMetaForCausalLM
+    keep = Ref.embed_video_streaming
     patched = flash_vstream_b200.install()
-    try:
-        from flash_vstream_b200 import compress_functions as mcf
-        assert rcf.weighted_kmeans_feature is mcf.weighted_kmeans_feature
-        assert rarch.weighted_kmeans_feature is mcf.weighted_kmeans_feature
-        assert "VStreamMetaForCausalLM.embed_video_streaming" in patched
-        assert rarch.VStreamMetaForCausalLM.embed_video_streaming is not keep[1]
-    finally:
-        import importlib
-        importlib.reload(rcf)
-        importlib.reload(rarch)
+    assert rcf.weighted_kmeans_feature is mcf.weighted_kmeans_feature
+    assert rarch.weighted_kmeans_feature is mcf.weighted_kmeans_feature
+    assert "VStreamMetaForCausalLM.embed_video_streaming" in patched
+    assert Ref.embed_video_streaming is not keep
+    for name in ref["modules"]["flash_vstream.model.compress_functions"]:
+        assert getattr(rcf, name) is getattr(mcf, name), name
+    assert rarch.build_vision_projector is mproj.build_vision_projector
+    assert mods["flash_vstream.model.multimodal_projector.builder"].build_vision_projector is mproj.build_vision_projector
+    for mod in ("flash_vstream.model.multimodal_encoder.clip_encoder", "flash_vstream.model.multimodal_encoder.builder"):
+        assert mods[mod].CLIPVisionTower is mclip.CLIPVisionTower, mod
+    for name in ("encode_images", "attention", "compress_spatial_features", "compress_temporal_features", "cat_proj",
+                 "reshape_2x2_image_features"):        # methods the original class defines and the mirror replaces
+        assert name in ref["VStreamMetaForCausalLM_methods"], name
+        assert getattr(Ref, name) is getattr(march.VStreamMetaForCausalLM, name), name
 
 
-QREF = "/root/reference/Flash-VStream-Qwen/models"
-
-
-@pytest.mark.skipif(not os.path.isdir(QREF), reason="reference tree only exists in the build container")
-def test_install_qwen_rebinds_reference_seam_and_signatures():
-    """the Qwen-side seam: FlashMemory (offline + streaming) and weighted_kmeans_ordered_feature on the reference's own
-    modules (imported with the harness shim of tests/golden/make_golden_qwen.py), same constructor / method signatures"""
-    import importlib
-    import types
-    import transformers.models.qwen2_vl.modeling_qwen2_vl as hf
-    if not hasattr(hf, "_prepare_4d_causal_attention_mask_with_cache_position"):
-        hf._prepare_4d_causal_attention_mask_with_cache_position = None
-    if "models" not in sys.modules:
-        pkg = types.ModuleType("models")
-        pkg.__path__ = [QREF]
-        sys.modules["models"] = pkg
-    ref_model = importlib.import_module("models.vstream_qwen2vl_model")
-    ref_rt = importlib.import_module("models.vstream_qwen2vl_realtime")
-    ref_cf = importlib.import_module("models.compress_functions")
+def test_install_qwen_rebinds_reference_seam_and_signatures(monkeypatch):
+    """the Qwen-side seam: FlashMemory (offline + streaming) and weighted_kmeans_ordered_feature on modules laid out like
+    the original `models.*` ones, same constructor / method signatures as the original's"""
     import flash_vstream_b200.qwen as mine
     from flash_vstream_b200.qwen import vstream_qwen2vl_realtime as mine_rt
-
-    def params(f):
-        return [(p.name, p.default) for p in inspect.signature(f).parameters.values() if p.kind is not p.KEYWORD_ONLY]
-
-    assert params(mine.FlashMemory.__init__) == params(ref_model.FlashMemory.__init__)
+    ref = _seams()["qwen"]
+    assert _params(mine.FlashMemory.__init__) == ref["FlashMemory"]["__init__"]
     for name in ("temporal_pool", "cat_spa_tem", "calc_am_rope"):
-        assert params(getattr(mine.FlashMemory, name)) == params(getattr(ref_model.FlashMemory, name)), name
+        assert _params(getattr(mine.FlashMemory, name)) == ref["FlashMemory"][name], name
     for name in ("temporal_compress", "spatial_enhance", "forward"):        # ours add one optional trailing `draws=None`
-        got = params(getattr(mine.FlashMemory, name))
-        assert got[:-1] == params(getattr(ref_model.FlashMemory, name)) and got[-1] == ("draws", None), name
-    got = params(mine_rt.FlashMemory.temporal_compress)
-    assert got[:-1] == params(ref_rt.FlashMemory.temporal_compress) and got[-1] == ("draws", None)
-    assert params(mine.weighted_kmeans_ordered_feature) == params(ref_cf.weighted_kmeans_ordered_feature)
-    for name in ("embed_new_video_clip", "prepare_realtime_inference", "get_video_embedding_memory_cuda_list"):
-        got = params(getattr(mine_rt.RealtimeStreamingMixin, name))
-        want = params(getattr(ref_rt.FlashVStreamQwen2VLModel, name))
+        got = _params(getattr(mine.FlashMemory, name))
+        assert got[:-1] == ref["FlashMemory"][name] and got[-1] == ["draws", "None"], name
+    got = _params(mine_rt.FlashMemory.temporal_compress)
+    assert got[:-1] == ref["realtime_FlashMemory"]["temporal_compress"] and got[-1] == ["draws", "None"]
+    assert _params(mine.weighted_kmeans_ordered_feature) == ref["weighted_kmeans_ordered_feature"]
+    for name, want in ref["FlashVStreamQwen2VLModel"].items():
+        got = _params(getattr(mine_rt.RealtimeStreamingMixin, name))
         assert got[: len(want)] == want, name
-    keep = (ref_model.FlashMemory, ref_rt.FlashMemory, ref_cf.weighted_kmeans_ordered_feature)
+    mods = _stand_in_modules(monkeypatch, ref["modules"])
+    ref_model, ref_rt = mods["models.vstream_qwen2vl_model"], mods["models.vstream_qwen2vl_realtime"]
+    ref_cf = mods["models.compress_functions"]
     from flash_vstream_b200.install import install_qwen
     patched = install_qwen()
-    try:
-        assert ref_model.FlashMemory is mine.FlashMemory and ref_rt.FlashMemory is mine_rt.FlashMemory
-        assert ref_cf.weighted_kmeans_ordered_feature is mine.weighted_kmeans_ordered_feature
-        assert len(patched) == 3
-    finally:
-        ref_model.FlashMemory, ref_rt.FlashMemory, ref_cf.weighted_kmeans_ordered_feature = keep
-        ref_model.weighted_kmeans_ordered_feature = keep[2]
-        ref_rt.weighted_kmeans_ordered_feature = keep[2]
+    assert ref_model.FlashMemory is mine.FlashMemory and ref_rt.FlashMemory is mine_rt.FlashMemory
+    assert ref_cf.weighted_kmeans_ordered_feature is mine.weighted_kmeans_ordered_feature
+    assert ref_model.weighted_kmeans_ordered_feature is mine.weighted_kmeans_ordered_feature
+    assert ref_rt.weighted_kmeans_ordered_feature is mine.weighted_kmeans_ordered_feature
+    assert len(patched) == 3
 
 
 def test_shard_streams():
@@ -340,3 +358,25 @@ def test_bench_gemm_breakdown_groups_launches_by_position():
     plain = (w[0] + 23 * 2.0 * M * (3072 + 4096) * 1024) / ((0.05 + 23 * 0.192) * 1e-3) / 1e12
     assert abs(out["without_residual_epilogue"] - plain) < 1e-6
     assert bench.gemm_breakdown(ms[:-1], w[:-1]) is None
+
+
+def test_bench_dump_outputs_writes_float32_memory_and_a_fixed_buffer_sample(tmp_path):
+    import importlib.util
+    import numpy as np
+    spec = importlib.util.spec_from_file_location("_bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    g = torch.Generator().manual_seed(0)
+    cur, lng, tur = (torch.randn(*s, generator=g).half() for s in ((4, 64, 32), (25, 16, 32), (25, 1, 32)))
+    buf = torch.arange(100, dtype=torch.float16).view(100, 1, 1).expand(100, 64, 32).contiguous()
+    names = bench.dump_outputs(str(tmp_path / "a"), [cur, lng, tur, buf], buffer_frames=8)
+    bench.dump_outputs(str(tmp_path / "b"), [cur, lng, tur, buf], buffer_frames=8)
+    assert names == ["memory_buffer_sample", "memory_current", "memory_long", "memory_turing"]
+    for name, want in (("memory_current", cur), ("memory_long", lng), ("memory_turing", tur)):
+        got = np.load(tmp_path / "a" / f"{name}.npy")
+        assert got.dtype == np.float32 and np.array_equal(got, want.float().numpy()), name
+    sample = np.load(tmp_path / "a" / "memory_buffer_sample.npy")
+    frames = sample[:, 0, 0]
+    assert sample.shape == (8, 64, 32) and sample.dtype == np.float32
+    assert len(set(frames)) == 8 and (np.diff(frames) > 0).all()          # distinct frames, in stream order
+    assert np.array_equal(sample, np.load(tmp_path / "b" / "memory_buffer_sample.npy"))   # the same frames every run
