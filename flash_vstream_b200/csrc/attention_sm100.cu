@@ -8,8 +8,7 @@
 //                 the packed [frames, tokens, 3*H*64] QKV activation by 3-D tensor maps; rows past `tokens` are
 //                 zero-filled by the TMA, so frames never bleed into each other)
 //   warp 1      : MMA issuer (converged warp, one elect.sync lane issues) — S_j = Q K_j^T into one of TWO TMEM score
-//                 buffers (S_{j+2} goes out as soon as S_j has been read);
-//                 O += P_j V_j (P K-major from smem, V MN-major straight from its TMA tile) and L += P_j 1 (row sums
+//                 buffers; O += P_j V_j (P from TMEM, V MN-major straight from its TMA tile) and L += P_j 1 (row sums
 //                 against a constant tile of ones) accumulate in TMEM
 //   warp 2      : TMEM allocator;  warp 3: builds the ones tile
 //   warps 4..11 : softmax, two threads per query row (warps 4-7: columns [0,32) of each 64-wide KV tile, warps 8-11:
@@ -19,44 +18,17 @@
 //                 the TMEM accumulators O|L are rescaled (tcgen05.ld/st read-modify-write) only when a tile raises the
 //                 maximum by more than 2^8, which after the first tile is rare.  The result is exact: O and L always
 //                 carry the same scale, and O/L is formed at the end.
+// P never touches shared memory: the softmax threads write the rounded P tile with tcgen05.st over the first 32 columns of
+// the S buffer they just drained, and the P V / row-sum MMAs take it as their TMEM A operand (tcgen05.mma [d], [a], b-desc).
+// S_{j+2} overwrites those columns, so the MMA issue order is S_0, S_1, then [P_j V_j, S_{j+2}] for j = 0, 1, ... in the
+// (in-order) tensor pipe.  That keeps the softmax chain free of shared-memory stores and proxy fences.  DESIGN.md §3.2 has
+// the measurements that chose this design over P in shared memory, a persistent schedule and the other variants that were
+// built, measured and removed.
 // tokens = 577 for ViT-L/14-336: 10 KV tiles, the last one 16 wide (1 valid key).
 // Replaces HF CLIPAttention reached from multimodal_encoder/clip_encoder.py:50 (SURVEY.md §2.2 K2).
 #include "fvs_common.h"
 #include "fvs_kernels.h"
 #include "fvs_ptx.cuh"
-
-#include <cstdlib>
-
-#ifndef FVS_ATTN_PERSIST_DEFAULT
-#define FVS_ATTN_PERSIST_DEFAULT 0   // flipped once the persistent kernel has been verified and measured on a B200
-#endif
-
-// FVS_ATTN_KNOCKOUT=n builds a deliberately WRONG one-shot kernel with one resource consumer removed, to measure which
-// resource bounds it (tests/ab_attn_knockout.sh): 1 no row-sum MMA, 2 no MUFU.EX2, 3 no P stores, 4 half the TMEM score
-// reads, 5 no P V / row-sum MMAs, 6 no row maximum / pair exchange.  Never defined in the product build.
-#ifndef FVS_ATTN_KNOCKOUT
-#define FVS_ATTN_KNOCKOUT 0
-#endif
-// FVS_ATTN_PTMEM=1 (default; one-shot kernel): P never touches shared memory — the softmax threads write the rounded P
-// tile with tcgen05.st over the first 32 columns of the S buffer they just drained, and P V / the row-sum MMA take it as
-// their TMEM A operand (tcgen05.mma [d], [a], b-desc).  S_{j+2} must then follow P_j V_j in the (in-order) tensor pipe, so
-// the issue order is [P_j V_j, S_{j+2}].  smem traffic per KV tile 98 -> 50 KB, no STS / proxy fence in the softmax chain.
-// Measured on one B200 against the smem-P build (profiles/r2_attn_variants.log): head_dim 64, 32 frames 117.9 -> 107.6 us
-// (370 -> 405 TFLOP/s), head_dim 80 35.4 -> 30.9 us (384 -> 439 TFLOP/s); bit-identical results.  =0 keeps P in smem
-// (what the persistent kernel and the knock-out builds use).  The other round-1 candidates were measured on the same box and
-// removed: row sums folded into P V (N = 80) and an elected-lane TMA producer were neutral, polynomial exp2 on the FMA pipe
-// was 5-8 % slower (the FMA pipe is busier than the SFU here).
-// Round-2 restructurings that were built, validated against torch and then REMOVED because they did not beat this kernel on
-// the same box (profiles/r2_attn_timeline.log has the per-CTA clock64 timelines): P in its own TMEM columns with S_{j+2}
-// issued ahead of P_j V_j (115 us: the extra pv_done wait costs more than the reordering gains — every mbarrier operation of a
-// softmax warp takes ~250 clk behind the MUFU instructions queued in the MIO pipe), one arrival per warp instead of per thread
-// (119 us), single-lane waits (218 us: a parked warp with one polling lane wakes up late), and a split-KV schedule with two
-// softmax groups on alternate KV tiles, one thread per row, two accumulators merged in the epilogue (110 us).  All of them
-// land at ~2.1 k clk per pair of 128 x 64 tiles per SM with the SFU 48 % busy: with 16 softmax warps per SM (TMEM and the
-// register file cap it at two CTAs) the exp / convert / hand-off chain of a warp is latency-bound, not pipe-bound.
-#ifndef FVS_ATTN_PTMEM
-#define FVS_ATTN_PTMEM 1
-#endif
 
 namespace fvs {
 namespace attn {
@@ -69,7 +41,7 @@ constexpr int kThreads = 384;
 constexpr int kSoftmaxThreads = 256;
 constexpr int Q_BYTES = BQ * HD * 2;      // 16 KB
 constexpr int KV_BYTES = BKV * HD * 2;    // 8 KB: [64 rows][64 x 16-bit], 128 B per row
-constexpr int P_BYTES = BQ * BKV * 2;     // 16 KB: [128 rows][64 x 16-bit]
+constexpr int STG_BYTES = BQ * HD * 2;    // 16 KB: [128 rows][64 x 16-bit] O tile staged for the TMA store
 constexpr int ONES_BYTES = 2048;          // [16 rows][64 x 16-bit] of 1.0 (B operand of the row-sum MMA)
 constexpr int XCHG_BYTES = 2 * 2 * 128 * 4;  // [tile parity][column group][row] partial maxima
 constexpr uint32_t TMEM_COLS = 256;  // S0: [0,64)  S1: [64,128)  O: [128,192) (+[192,208) extra dims)  L (row sums): 16 columns after O
@@ -80,7 +52,9 @@ constexpr int KVX_BYTES = BKV * XD * 2;   // 2 KB
 template <bool kX> struct Lay {
   static constexpr int Q_TOTAL = Q_BYTES + (kX ? QX_BYTES : 0);
   static constexpr int KV_STAGE = KV_BYTES + (kX ? KVX_BYTES : 0);     // 8 KB | 10 KB, both multiples of 1024
-  static constexpr int TILES = Q_TOTAL + kKVStages * KV_STAGE + 2 * P_BYTES + ONES_BYTES + XCHG_BYTES;
+  // The staging region is 2 * STG_BYTES although the O tile uses only its first half: the layout is kept byte-identical
+  // to the build that DESIGN.md §3.2 measured.
+  static constexpr int TILES = Q_TOTAL + kKVStages * KV_STAGE + 2 * STG_BYTES + ONES_BYTES + XCHG_BYTES;
   static constexpr int BYTES = TILES + 256 + 1024;
   static constexpr uint32_t L_OFF = kX ? 208 : 192;
 };
@@ -112,8 +86,8 @@ attention_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
   uint8_t* smem_q = smem;
   uint8_t* smem_qx = smem_q + Q_BYTES;                    // kX: [128][32 B] extra dims of Q (later: staging of the extra ctx dims)
   uint8_t* smem_kv = smem_q + L_::Q_TOTAL;                // [kKVStages][8 KB main (+ 2 KB extra)]
-  uint8_t* smem_p = smem_kv + kKVStages * L_::KV_STAGE;   // [2][16 KB]
-  uint8_t* smem_ones = smem_p + 2 * P_BYTES;              // 2 KB of 1.0
+  uint8_t* smem_stg = smem_kv + kKVStages * L_::KV_STAGE; // 16 KB O staging tile (+ 16 KB unused, see Lay)
+  uint8_t* smem_ones = smem_stg + 2 * STG_BYTES;          // 2 KB of 1.0
   float* smem_x = reinterpret_cast<float*>(smem_ones + ONES_BYTES);  // [2][2][128]
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + L_::TILES);
   uint64_t* q_full = bars;                 // 1
@@ -121,7 +95,7 @@ attention_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
   uint64_t* kv_empty = bars + 5;           // [4]
   uint64_t* s_full = bars + 9;             // [2] MMA -> softmax: S tile ready in TMEM buffer b
   uint64_t* s_empty = bars + 11;           // [2] softmax -> MMA: S buffer b drained to registers (256 arrivals)
-  uint64_t* p_full = bars + 13;            // [2] softmax -> MMA: P buffer b written (256 arrivals)
+  uint64_t* p_full = bars + 13;            // [2] softmax -> MMA: P written over S buffer b (256 arrivals)
   uint64_t* pv_done = bars + 15;           // [2] MMA -> softmax: P_j V_j (and everything before it) retired
   uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 17);
 
@@ -195,17 +169,12 @@ attention_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
       if (kX) tma_load_3d(smem_kv + stage * L_::KV_STAGE + KV_BYTES, &tmap_kvx, &kv_full[stage], xcol, row, frame);
       if (++stage == kKVStages) { stage = 0; phase ^= 1; }
     };
-    // consumption order of the MMA thread: K0, K1, then (K_{j+2}, V_j) for j = 0, 1, ...
+    // consumption order of the MMA thread: K0, K1, then (V_j, K_{j+2}) for j = 0, 1, ...
     load_tile(k_col, xk_col, 0);
     if (nkv > 1) load_tile(k_col, xk_col, BKV);
     for (int j = 0; j < nkv; ++j) {
-#if FVS_ATTN_PTMEM
       load_tile(v_col, xv_col, j * BKV);
       if (j + 2 < nkv) load_tile(k_col, xk_col, (j + 2) * BKV);
-#else
-      if (j + 2 < nkv) load_tile(k_col, xk_col, (j + 2) * BKV);
-      load_tile(v_col, xv_col, j * BKV);
-#endif
     }
   } else if (warp == 1) {
     // ------------------------------------------------------------------ MMA issuer
@@ -221,7 +190,7 @@ attention_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
     constexpr uint32_t idesc_s_full = umma_idesc_f16(BQ, BKV, kBF16, false, false);
     const uint32_t idesc_s_last = umma_idesc_f16(BQ, last_cols, kBF16, false, false);
     // descriptor words (see umma_desc_sw128 / umma_desc_sw32): hi = SBO | version | layout, lo = address >> 4 | LBO << 16
-    constexpr uint32_t HI_K = uint32_t(umma_desc_sw128(0, 1024, 16) >> 32);      // K-major SWIZZLE_128B (Q, K, P, ones)
+    constexpr uint32_t HI_K = uint32_t(umma_desc_sw128(0, 1024, 16) >> 32);      // K-major SWIZZLE_128B (Q, K, ones)
     constexpr uint32_t HI_V = uint32_t(umma_desc_sw128(0, 1024, 1024) >> 32);    // MN-major SWIZZLE_128B (V)
     constexpr uint32_t HI_X = uint32_t(umma_desc_sw32(0, 256, 256) >> 32);       // SWIZZLE_32B (extra dims)
     constexpr uint32_t LBO_K = uint32_t(umma_desc_sw128(0, 1024, 16));
@@ -232,7 +201,6 @@ attention_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
     const uint32_t qx_lo = (smem_u32(smem_qx) >> 4) | LBO_X;
     const uint32_t ones_lo = (smem_u32(smem_ones) >> 4) | LBO_K;
     const uint32_t kv_lo0 = smem_u32(smem_kv) >> 4;           // + stage * (KV_STAGE >> 4)
-    const uint32_t p_lo0 = (smem_u32(smem_p) >> 4) | LBO_K;   // + b * (P_BYTES >> 4)
     const uint32_t o_tmem = tmem_base + TMEM_O_OFF;
     const uint32_t l_tmem = tmem_base + TMEM_L_OFF;
     int stage = 0;
@@ -258,64 +226,42 @@ attention_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
       __syncwarp();
       if (++stage == kKVStages) { stage = 0; phase ^= 1; }
     };
-    auto issue_pv_step = [&](uint32_t p_lo, uint32_t v_lo, int k, uint32_t acc) {
-      // A = P[:, 16k..16k+16): K-major, 32-byte step inside the 128 B swizzle row; B = V[16k..16k+16, 0..64): MN-major,
-      // 16 kv rows = two 8-row groups (SBO = 1024 B apart), 2048 B per k step
-#if FVS_ATTN_PTMEM
-      {   // A = P[:, 16k..16k+16) from TMEM: 8 columns of packed pairs at the head of S buffer b (p_lo carries the address)
-        const uint32_t p_tmem = p_lo + 8 * k;
-        umma_f16_ts(o_tmem, p_tmem, desc((v_lo | LBO_V) + 128 * k, HI_V), idesc_pv, acc);
-        if (kX) umma_f16_ts(o_tmem + HD, p_tmem, desc(((v_lo + (KV_BYTES >> 4)) | LBO_X) + 32 * k, HI_X), idesc_pvx, acc);
-        umma_f16_ts(l_tmem, p_tmem, desc(ones_lo, HI_K), idesc_l, acc);
-        return;
-      }
-#endif
-      const uint64_t p_desc = desc(p_lo + 2 * k, HI_K);
-#if FVS_ATTN_KNOCKOUT != 5
-      umma_f16_ss(o_tmem, p_desc, desc((v_lo | LBO_V) + 128 * k, HI_V), idesc_pv, acc);
-#endif
+    auto issue_pv_step = [&](uint32_t p_tmem, uint32_t v_lo, int k, uint32_t acc) {
+      // A = P[:, 16k..16k+16) from TMEM: 8 columns of packed pairs at the head of S buffer b; B = V[16k..16k+16, 0..64):
+      // MN-major, 16 kv rows = two 8-row groups (SBO = 1024 B apart), 2048 B per k step
+      const uint32_t a_tmem = p_tmem + 8 * k;
+      umma_f16_ts(o_tmem, a_tmem, desc((v_lo | LBO_V) + 128 * k, HI_V), idesc_pv, acc);
       if (kX)   // O[:, 64..80) += P V_extra: B = V_extra[16k..16k+16, 0..16) MN-major, two 8-row groups 256 B apart
-        umma_f16_ss(o_tmem + HD, p_desc, desc(((v_lo + (KV_BYTES >> 4)) | LBO_X) + 32 * k, HI_X), idesc_pvx, acc);
-#if FVS_ATTN_KNOCKOUT != 1 && FVS_ATTN_KNOCKOUT != 5
-      umma_f16_ss(l_tmem, p_desc, desc(ones_lo, HI_K), idesc_l, acc);  // row sums of the rounded P
-#endif
+        umma_f16_ts(o_tmem + HD, a_tmem, desc(((v_lo + (KV_BYTES >> 4)) | LBO_X) + 32 * k, HI_X), idesc_pvx, acc);
+      umma_f16_ts(l_tmem, a_tmem, desc(ones_lo, HI_K), idesc_l, acc);  // row sums of the rounded P
     };
 
-    // Issue order: S_{j+2} goes out as soon as the softmax warps have pulled S_j out of its TMEM buffer (early in their
-    // work on tile j), NOT behind P_j V_j: the P -> P V -> pv_done hand-off has two tiles of slack.
+    // Issue order: S_0, S_1, then [P_j V_j, S_{j+2}]: S_{j+2} overwrites the TMEM columns P_j lives in, so it has to
+    // follow P_j V_j in the (in-order) tensor pipe.
     mbar_wait(q_full, 0);
     issue_s(0);
     if (nkv > 1) issue_s(1);
     for (int j = 0; j < nkv; ++j) {
-#if !FVS_ATTN_PTMEM
-      if (j + 2 < nkv) issue_s(j + 2);
-#endif
       const int b = j & 1;
       mbar_wait(&kv_full[stage], phase);          // V_j landed
       mbar_wait(&p_full[b], (j >> 1) & 1);        // P_j written (and any O|L rescale finished)
       tc_fence_after_sync();
       const uint32_t v_lo = kv_lo0 + stage * (L_::KV_STAGE >> 4);
-#if FVS_ATTN_PTMEM
-      const uint32_t p_lo = tmem_base + b * BKV;  // TMEM address of P_j (aliases the drained S buffer)
-#else
-      const uint32_t p_lo = p_lo0 + b * (P_BYTES >> 4);
-#endif
+      const uint32_t p_tmem = tmem_base + b * BKV;  // TMEM address of P_j (aliases the drained S buffer)
       if (elect_one()) {
         if (j < nkv - 1 || last_cols == BKV) {
-          issue_pv_step(p_lo, v_lo, 0, j != 0 ? 1u : 0u);
+          issue_pv_step(p_tmem, v_lo, 0, j != 0 ? 1u : 0u);
 #pragma unroll
-          for (int k = 1; k < BKV / 16; ++k) issue_pv_step(p_lo, v_lo, k, 1u);
+          for (int k = 1; k < BKV / 16; ++k) issue_pv_step(p_tmem, v_lo, k, 1u);
         } else {
-          for (int k = 0; k < last_cols / 16; ++k) issue_pv_step(p_lo, v_lo, k, (j | k) != 0 ? 1u : 0u);
+          for (int k = 0; k < last_cols / 16; ++k) issue_pv_step(p_tmem, v_lo, k, (j | k) != 0 ? 1u : 0u);
         }
         umma_commit(&kv_empty[stage]);
         umma_commit(&pv_done[b]);
       }
       __syncwarp();
       if (++stage == kKVStages) { stage = 0; phase ^= 1; }
-#if FVS_ATTN_PTMEM
       if (j + 2 < nkv) issue_s(j + 2);            // behind P_j V_j: S_{j+2} overwrites the TMEM columns P_j lives in
-#endif
     }
   } else if (warp >= 4) {
     // ------------------------------------------------------------------ softmax: 2 threads per query row
@@ -325,10 +271,6 @@ attention_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
     const int rsw = r & 7;                    // swizzle phase of this row
     const uint32_t lane_addr = uint32_t(quad * 32) << 16;
     float m_run = -INFINITY;                  // running row maximum of the raw scores (identical in both threads of a row)
-    // byte offsets of this thread's four 16-byte P chunks inside a P buffer (row r, chunks 4*grp .. 4*grp+3, swizzled)
-    uint32_t pchunk[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) pchunk[i] = uint32_t(r * 128 + (((grp * 4 + i) ^ rsw) << 4));
     float* const xs_mine = smem_x + grp * 128 + r;
     float* const xs_peer = smem_x + (grp ^ 1) * 128 + r;
     const uint32_t s_addr0 = tmem_base + lane_addr + grp * 32;
@@ -342,18 +284,8 @@ attention_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
       mbar_wait(&s_full[b], (j >> 1) & 1);
       tc_fence_after_sync();
       uint32_t v[32];
-#if FVS_ATTN_KNOCKOUT == 4
-      {
-        uint32_t h[16];
-        tmem_ld_32x32b_x16(s_addr0 + b * BKV, h);
-        tmem_ld_wait_dep(h);
-#pragma unroll
-        for (int e = 0; e < 16; ++e) { v[e] = h[e]; v[16 + e] = h[e] ^ 0x00010000u; }
-      }
-#else
       tmem_ld_32x32b_x32(s_addr0 + b * BKV, v);
       tmem_ld_wait_dep(v);
-#endif
       tc_fence_before_sync();
       mbar_arrive(&s_empty[b]);               // S buffer b may be overwritten by S_{j+2}
 
@@ -366,15 +298,11 @@ attention_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
           if (e >= myvalid) v[e] = 0xff800000u;   // -inf
       }
       float tmax = -INFINITY;
-#if FVS_ATTN_KNOCKOUT == 6
-      tmax = 8.0f;
-#else
 #pragma unroll
       for (int e = 0; e < 32; ++e) tmax = fmaxf(tmax, __uint_as_float(v[e]));
       xs_mine[b * 256] = tmax;                // exchange slot of this tile parity
       named_bar_sync(2 + quad, 64);           // the two warps that share these 32 rows
       tmax = fmaxf(tmax, xs_peer[b * 256]);
-#endif
 
       // ---- lazy rescale of the TMEM accumulators
       const bool grow = (tmax - m_run) * scale_log2e > kRescaleThreshold;  // true at j == 0 (m_run = -inf)
@@ -405,10 +333,11 @@ attention_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
         m_run = m_new;
       }
 
-#if FVS_ATTN_PTMEM
       // ---- P_j = exp2((S - m_run) * scale*log2e) -> TMEM, packed pairs over the head of S buffer b (this thread's 32 columns
       // -> 16 TMEM columns at 16 * grp).  The partner thread of the row has loaded ITS scores before the pair barrier above,
-      // so overwriting its columns is safe; S_{j+2} is only issued behind P_j V_j.
+      // so overwriting its columns is safe; S_{j+2} is only issued behind P_j V_j.  Masked columns carry -inf, so ex2 gives
+      // exactly 0 (no separate masking pass); a thread with no valid column at all (second column group of a narrow last
+      // tile) just writes zeros.
       {
         const float neg_max_scaled = -m_run * scale_log2e;
         uint32_t w[16];
@@ -420,46 +349,11 @@ attention_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
         tmem_st_32x32b_x16(tmem_base + lane_addr + b * BKV + grp * 16, w);
         tmem_st_wait();
       }
-      tc_fence_before_sync();
+      tc_fence_before_sync();                 // orders the tcgen05.st of P and of a rescale before the MMA thread's P V
       mbar_arrive(&p_full[b]);
-#else
-      // ---- P_j = exp2((S - m_run) * scale*log2e) -> P buffer b (16-bit, SWIZZLE_128B K-major)
-      if (j >= 2) mbar_wait(&pv_done[b], ((j - 2) >> 1) & 1);   // P V_{j-2} no longer reads this buffer
-      {
-        const float neg_max_scaled = -m_run * scale_log2e;
-        uint8_t* pbuf = smem_p + b * P_BYTES;
-        // masked columns carry -inf -> ex2 gives exactly 0 (no separate masking pass); a thread with no valid column at all
-        // (second column group of a narrow last tile) just stores zeros
-        if (myvalid <= 0) {
-#pragma unroll
-          for (int i = 0; i < 4; ++i) *reinterpret_cast<uint4*>(pbuf + pchunk[i]) = make_uint4(0u, 0u, 0u, 0u);
-        } else {
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {       // 4 x (8 columns = 16 bytes)
-            uint32_t w[4];
-#pragma unroll
-            for (int e = 0; e < 8; e += 2)
-#if FVS_ATTN_KNOCKOUT == 2
-              w[e >> 1] = pack2<kBF16>(fmaf(__uint_as_float(v[i * 8 + e]), scale_log2e, neg_max_scaled),
-                                       fmaf(__uint_as_float(v[i * 8 + e + 1]), scale_log2e, neg_max_scaled));
-#else
-              w[e >> 1] = pack2<kBF16>(ex2_approx(fmaf(__uint_as_float(v[i * 8 + e]), scale_log2e, neg_max_scaled)),
-                                       ex2_approx(fmaf(__uint_as_float(v[i * 8 + e + 1]), scale_log2e, neg_max_scaled)));
-#endif
-#if FVS_ATTN_KNOCKOUT == 3
-            if (w[0] == 0x12345678u)   // never true in practice: keeps the arithmetic alive without the store traffic
-#endif
-            *reinterpret_cast<uint4*>(pbuf + pchunk[i]) = make_uint4(w[0], w[1], w[2], w[3]);
-          }
-        }
-      }
-      tc_fence_before_sync();                 // orders the tcgen05.st of a rescale before the MMA thread's next P V
-      fence_proxy_async_smem();
-      mbar_arrive(&p_full[b]);
-#endif
     }
 
-    // ---- epilogue: O / L -> 16-bit -> swizzled staging (reuses P buffer 0) -> TMA store; each thread 32 of the 64 dims
+    // ---- epilogue: O / L -> 16-bit -> swizzled staging tile -> TMA store; each thread 32 of the 64 dims
     mbar_wait(&pv_done[(nkv - 1) & 1], ((nkv - 1) >> 1) & 1);
     tc_fence_after_sync();
     uint32_t o[32], lsum[16];
@@ -468,7 +362,7 @@ attention_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
     tmem_ld_wait_dep(o);
     tmem_ld_wait_dep(lsum);
     const float inv = 1.0f / __uint_as_float(lsum[0]);
-    uint8_t* stg = smem_p + r * 128;
+    uint8_t* stg = smem_stg + r * 128;
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
       uint4 w;
@@ -495,7 +389,7 @@ attention_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
     fence_proxy_async_smem();
     named_bar_sync(1, kSoftmaxThreads);
     if (threadIdx.x == 128) {
-      tma_store_3d(&tmap_ctx, smem_p, head * HD, q0, frame);  // rows >= tokens are clipped by the map
+      tma_store_3d(&tmap_ctx, smem_stg, head * HD, q0, frame);  // rows >= tokens are clipped by the map
       if (kX) tma_store_3d(&tmap_ctxx, smem_qx, heads * HD + head * XD, q0, frame);
       tma_store_commit();
       tma_store_wait_all<0>();
@@ -509,401 +403,6 @@ attention_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
     tmem_dealloc<TMEM_COLS>(tmem_base);
   }
 }
-
-
-// ---------------------------------------------------------------------------------------------------------------------
-// Persistent variant.  The one-shot kernel above pays, per (query tile, head, frame) item, a serial prologue (barrier
-// init, TMEM allocation, first Q/K TMA round trip, first S MMA) and epilogue (O read-out, TMA store drain, TMEM
-// release) during which its softmax warps idle: the ncu source view of the one-shot kernel puts ~30 % of the softmax
-// warps' samples on the very first wait for S.  Here 2 CTAs per SM stay resident and walk over their items
-// (item = blockIdx.x + k * gridDim.x, query tile fastest so that co-scheduled CTAs share one head's K/V in L2) with every
-// ring — K/V stages, S/P double buffers and their mbarrier phases — running straight across item boundaries:
-//   * the TMA producer and the MMA issuer look ahead INTO THE NEXT ITEM exactly as they look ahead inside one: the flat
-//     tile order is S_0 S_1 [S_{g+2} PV_g]..., so S_0/S_1 of the next item are issued under the last two softmax tiles of
-//     the current one and the softmax warps find their first scores waiting;
-//   * Q is double-buffered (single-buffered for head_dim 80, whose tiles leave no room; its reload is released by the
-//     commit of the item's last S MMA, two tiles before the item ends);
-//   * the epilogue stages O/L in the P buffer that the next item touches SECOND and hands it to an otherwise idle
-//     service warp (warp 3), which issues the TMA store and signals `stg_free` once the bulk read has drained; the softmax
-//     warps only look at that barrier right before they overwrite the buffer (next item's tile 1), so the store never sits
-//     on their critical path;
-//   * PV_0 of the next item (accumulate = 0) is ordered after every thread's O/L read-out by the P_0 handshake itself:
-//     p_full needs all 256 softmax threads, and each arrives only after its own tcgen05.wait::ld + fence.
-template <bool kX> struct PLay {
-  static constexpr int kQB = kX ? 1 : 2;                               // Q buffers
-  static constexpr int STGX = kX ? QX_BYTES : 0;                       // staging of the 16 extra ctx dims
-  static constexpr int TILES = kQB * Lay<kX>::Q_TOTAL + kKVStages * Lay<kX>::KV_STAGE + 2 * P_BYTES + ONES_BYTES +
-                               XCHG_BYTES + STGX;
-  static constexpr int BYTES = TILES + 256 + 1024;
-};
-
-template <bool kBF16, bool kX>
-__global__ void __launch_bounds__(kThreads, 2)
-attention_persistent_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_kv,
-                            const __grid_constant__ CUtensorMap tmap_ctx, const __grid_constant__ CUtensorMap tmap_qx,
-                            const __grid_constant__ CUtensorMap tmap_kvx, const __grid_constant__ CUtensorMap tmap_ctxx,
-                            int tokens, int heads, int frames, float scale_log2e) {
-  using L_ = Lay<kX>;
-  using P_ = PLay<kX>;
-  constexpr int kQB = P_::kQB;
-  constexpr uint32_t TMEM_L_OFF = L_::L_OFF;
-  extern __shared__ __align__(1024) uint8_t smem[];
-  if ((smem_u32(smem) & 1023u) != 0) __trap();
-  uint8_t* smem_q = smem;                                  // [kQB][16 KB main (+ 4 KB extra)]
-  uint8_t* smem_kv = smem_q + kQB * L_::Q_TOTAL;           // [kKVStages][8 KB main (+ 2 KB extra)]
-  uint8_t* smem_p = smem_kv + kKVStages * L_::KV_STAGE;    // [2][16 KB]
-  uint8_t* smem_ones = smem_p + 2 * P_BYTES;               // 2 KB of 1.0
-  float* smem_x = reinterpret_cast<float*>(smem_ones + ONES_BYTES);  // [2][2][128]
-  uint8_t* smem_stgx = smem_ones + ONES_BYTES + XCHG_BYTES;          // kX: [128][32 B] extra ctx dims (SWIZZLE_32B)
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + P_::TILES);
-  uint64_t* q_full = bars;                 // [2] TMA -> MMA
-  uint64_t* q_empty = bars + 2;            // [2] MMA (commit of the item's last S) -> TMA
-  uint64_t* kv_full = bars + 4;            // [4]
-  uint64_t* kv_empty = bars + 8;           // [4]
-  uint64_t* s_full = bars + 12;            // [2] MMA -> softmax
-  uint64_t* s_empty = bars + 14;           // [2] softmax -> MMA (256 arrivals)
-  uint64_t* p_full = bars + 16;            // [2] softmax -> MMA (256 arrivals)
-  uint64_t* pv_done = bars + 18;           // [2] MMA -> softmax
-  uint64_t* stg_full = bars + 20;          // softmax -> store warp: O staged (256 arrivals), one phase per item
-  uint64_t* stg_free = bars + 21;          // store warp -> softmax: the TMA store has read the staging buffer
-  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 22);
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  const int nq = (tokens + BQ - 1) / BQ;
-  const int total = nq * heads * frames;                     // gridDim.x <= total
-  const int n_items = (total - int(blockIdx.x) + int(gridDim.x) - 1) / int(gridDim.x);
-  const int nkv = (tokens + BKV - 1) / BKV;
-  const int last_cols = ((tokens - (nkv - 1) * BKV) + 15) & ~15;  // width of the last KV tile, multiple of 16
-  const int n_tiles = n_items * nkv;                         // flat tile index g = it * nkv + j
-
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&tmap_q);
-    tma_prefetch_desc(&tmap_kv);
-    tma_prefetch_desc(&tmap_ctx);
-  }
-  if (warp == 1 && lane == 0) {
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&q_full[i], 1);
-      mbar_init(&q_empty[i], 1);
-      mbar_init(&s_full[i], 1);
-      mbar_init(&s_empty[i], kSoftmaxThreads);
-      mbar_init(&p_full[i], kSoftmaxThreads);
-      mbar_init(&pv_done[i], 1);
-    }
-    for (int s = 0; s < kKVStages; ++s) {
-      mbar_init(&kv_full[s], 1);
-      mbar_init(&kv_empty[s], 1);
-    }
-    mbar_init(stg_full, kSoftmaxThreads);
-    mbar_init(stg_free, 1);
-    fence_mbar_init();
-  }
-  if (warp == 2) {
-    tmem_alloc<TMEM_COLS>(tmem_ptr_smem);
-    tmem_relinquish();
-  }
-  if (warp == 3) {
-    const uint32_t one2 = kBF16 ? 0x3F803F80u : 0x3C003C00u;
-    for (int i = lane; i < ONES_BYTES / 16; i += 32)
-      reinterpret_cast<uint4*>(smem_ones)[i] = make_uint4(one2, one2, one2, one2);
-    fence_proxy_async_smem();
-  }
-  tc_fence_before_sync();
-  __syncthreads();
-  tc_fence_after_sync();
-  const uint32_t tmem_base = *tmem_ptr_smem;
-
-  if (warp < 4) reg_dealloc<64>(); else reg_alloc<88>();
-
-  pdl_trigger();
-  pdl_wait();
-
-  // item `it` of this CTA -> (first query row, head, frame)
-  auto coords = [&](int it, int& q0, int& head, int& frame) {
-    const int item = int(blockIdx.x) + it * int(gridDim.x);
-    const int hf = item / nq;
-    q0 = (item - hf * nq) * BQ;
-    frame = hf / heads;
-    head = hf - frame * heads;
-  };
-
-  if (warp == 0 && lane == 0) {
-    // ------------------------------------------------------------------ TMA producer
-    int stage = 0;
-    uint32_t phase = 0;
-    auto ring_load = [&](int col, int xcol, int row, int frame) {
-      mbar_wait(&kv_empty[stage], phase ^ 1);
-      mbar_arrive_expect_tx(&kv_full[stage], L_::KV_STAGE);
-      tma_load_3d(smem_kv + stage * L_::KV_STAGE, &tmap_kv, &kv_full[stage], col, row, frame);
-      if (kX) tma_load_3d(smem_kv + stage * L_::KV_STAGE + KV_BYTES, &tmap_kvx, &kv_full[stage], xcol, row, frame);
-      if (++stage == kKVStages) { stage = 0; phase ^= 1; }
-    };
-    auto load_k = [&](int g) {   // K tile of flat tile g; the first tile of an item brings the item's Q along
-      const int it = g / nkv, j = g - it * nkv;
-      int q0, head, frame;
-      coords(it, q0, head, frame);
-      if (j == 0) {
-        const int qb = it % kQB, use = it / kQB;
-        mbar_wait(&q_empty[qb], (use & 1) ^ 1);             // previous occupant's last S MMA has retired
-        mbar_arrive_expect_tx(&q_full[qb], L_::Q_TOTAL);
-        tma_load_3d(smem_q + qb * L_::Q_TOTAL, &tmap_q, &q_full[qb], head * HD, q0, frame);
-        if (kX) tma_load_3d(smem_q + qb * L_::Q_TOTAL + Q_BYTES, &tmap_qx, &q_full[qb], 3 * heads * HD + head * XD, q0, frame);
-      }
-      ring_load(heads * HD + head * HD, 3 * heads * HD + heads * XD + head * XD, j * BKV, frame);
-    };
-    auto load_v = [&](int g) {
-      const int it = g / nkv, j = g - it * nkv;
-      int q0, head, frame;
-      coords(it, q0, head, frame);
-      ring_load(2 * heads * HD + head * HD, 3 * heads * HD + 2 * heads * XD + head * XD, j * BKV, frame);
-    };
-    // consumption order of the MMA thread: K_0, K_1, then (K_{g+2}, V_g) for g = 0, 1, ... across item boundaries
-    load_k(0);
-    if (n_tiles > 1) load_k(1);
-    for (int g = 0; g < n_tiles; ++g) {
-      if (g + 2 < n_tiles) load_k(g + 2);
-      load_v(g);
-    }
-  } else if (warp == 1) {
-    // ------------------------------------------------------------------ MMA issuer: whole warp in the control flow, one
-    // elected lane issues, descriptors as (lo, hi) words in the uniform datapath (see the one-shot kernel)
-    constexpr uint32_t idesc_pv = umma_idesc_f16(BQ, HD, kBF16, false, /*B = V is MN-major*/ true);
-    constexpr uint32_t idesc_l = umma_idesc_f16(BQ, 16, kBF16, false, false);
-    constexpr uint32_t idesc_pvx = umma_idesc_f16(BQ, XD, kBF16, false, /*B = V extra is MN-major*/ true);
-    constexpr uint32_t idesc_s_full = umma_idesc_f16(BQ, BKV, kBF16, false, false);
-    const uint32_t idesc_s_last = umma_idesc_f16(BQ, last_cols, kBF16, false, false);
-    constexpr uint32_t HI_K = uint32_t(umma_desc_sw128(0, 1024, 16) >> 32);
-    constexpr uint32_t HI_V = uint32_t(umma_desc_sw128(0, 1024, 1024) >> 32);
-    constexpr uint32_t HI_X = uint32_t(umma_desc_sw32(0, 256, 256) >> 32);
-    constexpr uint32_t LBO_K = uint32_t(umma_desc_sw128(0, 1024, 16));
-    constexpr uint32_t LBO_V = uint32_t(umma_desc_sw128(0, 1024, 1024));
-    constexpr uint32_t LBO_X = uint32_t(umma_desc_sw32(0, 256, 256));
-    auto desc = [](uint32_t lo, uint32_t hi) { return (uint64_t(hi) << 32) | lo; };
-    const uint32_t q_lo0 = smem_u32(smem_q) >> 4;             // + qb * (Q_TOTAL >> 4)
-    const uint32_t ones_lo = (smem_u32(smem_ones) >> 4) | LBO_K;
-    const uint32_t kv_lo0 = smem_u32(smem_kv) >> 4;           // + stage * (KV_STAGE >> 4)
-    const uint32_t p_lo0 = (smem_u32(smem_p) >> 4) | LBO_K;   // + b * (P_BYTES >> 4)
-    const uint32_t o_tmem = tmem_base + TMEM_O_OFF;
-    const uint32_t l_tmem = tmem_base + TMEM_L_OFF;
-    int stage = 0;
-    uint32_t phase = 0;
-
-    int s_it = 0, s_j = 0;       // (item, tile) of the next S to issue; the P V loop below carries its own tile counter
-    auto issue_s = [&](int g) {  // S of flat tile g = s_it * nkv + s_j -> TMEM buffer (g & 1)
-      const int it = s_it, j = s_j;
-      const int qb = it % kQB;
-      const int b = g & 1;
-      if (j == 0) mbar_wait(&q_full[qb], (it / kQB) & 1);
-      mbar_wait(&kv_full[stage], phase);
-      if (g >= 2) mbar_wait(&s_empty[b], ((g - 2) >> 1) & 1);  // softmax has drained tile g-2 from this buffer
-      tc_fence_after_sync();
-      const uint32_t idesc_s = (j == nkv - 1) ? idesc_s_last : idesc_s_full;
-      const uint32_t q_lo = q_lo0 + qb * (L_::Q_TOTAL >> 4);
-      const uint32_t k_lo = kv_lo0 + stage * (L_::KV_STAGE >> 4);
-      const uint32_t s_tmem = tmem_base + b * BKV;
-      if (elect_one()) {
-#pragma unroll
-        for (int k = 0; k < HD / 16; ++k)
-          umma_f16_ss(s_tmem, desc((q_lo | LBO_K) + 2 * k, HI_K), desc((k_lo | LBO_K) + 2 * k, HI_K), idesc_s, k != 0 ? 1u : 0u);
-        if (kX)
-          umma_f16_ss(s_tmem, desc((q_lo + (Q_BYTES >> 4)) | LBO_X, HI_X), desc((k_lo + (KV_BYTES >> 4)) | LBO_X, HI_X), idesc_s, 1u);
-        umma_commit(&kv_empty[stage]);
-        umma_commit(&s_full[b]);
-        if (j == nkv - 1) umma_commit(&q_empty[qb]);          // the item's Q is dead: the producer may reload this buffer
-      }
-      __syncwarp();
-      if (++stage == kKVStages) { stage = 0; phase ^= 1; }
-      if (++s_j == nkv) { s_j = 0; ++s_it; }
-    };
-    auto issue_pv_step = [&](uint32_t p_lo, uint32_t v_lo, int k, uint32_t acc) {
-      const uint64_t p_desc = desc(p_lo + 2 * k, HI_K);
-      umma_f16_ss(o_tmem, p_desc, desc((v_lo | LBO_V) + 128 * k, HI_V), idesc_pv, acc);
-      if (kX)
-        umma_f16_ss(o_tmem + HD, p_desc, desc(((v_lo + (KV_BYTES >> 4)) | LBO_X) + 32 * k, HI_X), idesc_pvx, acc);
-      umma_f16_ss(l_tmem, p_desc, desc(ones_lo, HI_K), idesc_l, acc);  // row sums of the rounded P
-    };
-
-    issue_s(0);
-    if (n_tiles > 1) issue_s(1);
-    for (int g = 0, j = 0; g < n_tiles; ++g, j = (j + 1 == nkv) ? 0 : j + 1) {
-      if (g + 2 < n_tiles) issue_s(g + 2);        // as soon as tile g's scores have left their TMEM buffer
-      const int b = g & 1;
-      mbar_wait(&kv_full[stage], phase);          // V landed
-      mbar_wait(&p_full[b], (g >> 1) & 1);        // P written (any O|L rescale finished; at j == 0: previous O|L read out)
-      tc_fence_after_sync();
-      const uint32_t v_lo = kv_lo0 + stage * (L_::KV_STAGE >> 4);
-      const uint32_t p_lo = p_lo0 + b * (P_BYTES >> 4);
-      if (elect_one()) {
-        if (j < nkv - 1 || last_cols == BKV) {
-          issue_pv_step(p_lo, v_lo, 0, j != 0 ? 1u : 0u);
-#pragma unroll
-          for (int k = 1; k < BKV / 16; ++k) issue_pv_step(p_lo, v_lo, k, 1u);
-        } else {
-          for (int k = 0; k < last_cols / 16; ++k) issue_pv_step(p_lo, v_lo, k, (j | k) != 0 ? 1u : 0u);
-        }
-        umma_commit(&kv_empty[stage]);
-        umma_commit(&pv_done[b]);
-      }
-      __syncwarp();
-      if (++stage == kKVStages) { stage = 0; phase ^= 1; }
-    }
-  } else if (warp == 3 && lane == 0) {
-    // ------------------------------------------------------------------ store warp: staged O tile -> global
-    for (int it = 0; it < n_items; ++it) {
-      int q0, head, frame;
-      coords(it, q0, head, frame);
-      const int sb = (it * nkv + nkv - 1) & 1;     // P buffer of the item's last tile = the one the next item uses second
-      mbar_wait(stg_full, it & 1);                 // every writer fenced its st.shared towards the async proxy before arriving
-      tma_store_3d(&tmap_ctx, smem_p + sb * P_BYTES, head * HD, q0, frame);   // rows >= tokens are clipped by the map
-      if (kX) tma_store_3d(&tmap_ctxx, smem_stgx, heads * HD + head * XD, q0, frame);
-      tma_store_commit();
-      tma_store_wait_read<0>();
-      mbar_arrive(stg_free);
-    }
-    tma_store_wait_all<0>();
-  } else if (warp >= 4) {
-    // ------------------------------------------------------------------ softmax: 2 threads per query row
-    const int quad = warp & 3;
-    const int grp = (warp - 4) >> 2;
-    const int r = quad * 32 + lane;
-    const int rsw = r & 7;
-    const uint32_t lane_addr = uint32_t(quad * 32) << 16;
-    uint32_t pchunk[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) pchunk[i] = uint32_t(r * 128 + (((grp * 4 + i) ^ rsw) << 4));
-    float* const xs_mine = smem_x + grp * 128 + r;
-    float* const xs_peer = smem_x + (grp ^ 1) * 128 + r;
-    const uint32_t s_addr0 = tmem_base + lane_addr + grp * 32;
-    int g = 0;
-
-    for (int it = 0; it < n_items; ++it) {
-      float m_run = -INFINITY;
-      for (int j = 0; j < nkv; ++j, ++g) {
-        const int b = g & 1;
-        const int myvalid = tokens - j * BKV - grp * 32;
-        mbar_wait(&s_full[b], (g >> 1) & 1);
-        tc_fence_after_sync();
-        uint32_t v[32];
-        tmem_ld_32x32b_x32(s_addr0 + b * BKV, v);
-        tmem_ld_wait_dep(v);
-        tc_fence_before_sync();
-        mbar_arrive(&s_empty[b]);
-
-        const bool full = myvalid >= 32;
-        if (!full) {
-#pragma unroll
-          for (int e = 0; e < 32; ++e)
-            if (e >= myvalid) v[e] = 0xff800000u;   // -inf
-        }
-        float tmax = -INFINITY;
-#pragma unroll
-        for (int e = 0; e < 32; ++e) tmax = fmaxf(tmax, __uint_as_float(v[e]));
-        xs_mine[b * 256] = tmax;
-        named_bar_sync(2 + quad, 64);
-        tmax = fmaxf(tmax, xs_peer[b * 256]);
-
-        const bool grow = (tmax - m_run) * scale_log2e > kRescaleThreshold;
-        if (j == 0) {
-          m_run = tmax;
-        } else if (__any_sync(0xffffffffu, grow)) {
-          const float m_new = grow ? tmax : m_run;
-          const float factor = grow ? ex2_approx((m_run - m_new) * scale_log2e) : 1.0f;
-          mbar_wait(&pv_done[(g - 1) & 1], ((g - 1) >> 1) & 1);
-          tc_fence_after_sync();
-          const uint32_t o_addr = tmem_base + lane_addr + TMEM_O_OFF + grp * 32;
-#pragma unroll 1
-          for (int h = 0; h < 3; ++h) {
-            if (h == 2 && grp != 0 && !kX) break;
-            const uint32_t a = (h < 2) ? o_addr + h * 16
-                                       : tmem_base + lane_addr + (grp == 0 ? TMEM_L_OFF : TMEM_O_OFF + HD);
-            uint32_t o[16];
-            tmem_ld_32x32b_x16(a, o);
-            tmem_ld_wait_dep(o);
-#pragma unroll
-            for (int e = 0; e < 16; ++e) o[e] = __float_as_uint(__uint_as_float(o[e]) * factor);
-            tmem_st_32x32b_x16(a, o);
-          }
-          tmem_st_wait();
-          m_run = m_new;
-        }
-
-        if (g >= 2) mbar_wait(&pv_done[b], ((g - 2) >> 1) & 1);   // P V of tile g-2 no longer reads this buffer
-        // ... nor does the previous item's TMA store: it was staged in the buffer of that item's last tile, which is
-        // this item's tile 1 (single-tile items wait in their epilogue instead)
-        if (j == 1 && it > 0) mbar_wait(stg_free, (it - 1) & 1);
-        {
-          const float neg_max_scaled = -m_run * scale_log2e;
-          uint8_t* pbuf = smem_p + b * P_BYTES;
-          if (myvalid <= 0) {
-#pragma unroll
-            for (int i = 0; i < 4; ++i) *reinterpret_cast<uint4*>(pbuf + pchunk[i]) = make_uint4(0u, 0u, 0u, 0u);
-          } else {
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-              uint32_t w[4];
-#pragma unroll
-              for (int e = 0; e < 8; e += 2)
-                w[e >> 1] = pack2<kBF16>(ex2_approx(fmaf(__uint_as_float(v[i * 8 + e]), scale_log2e, neg_max_scaled)),
-                                         ex2_approx(fmaf(__uint_as_float(v[i * 8 + e + 1]), scale_log2e, neg_max_scaled)));
-              *reinterpret_cast<uint4*>(pbuf + pchunk[i]) = make_uint4(w[0], w[1], w[2], w[3]);
-            }
-          }
-        }
-        tc_fence_before_sync();
-        fence_proxy_async_smem();
-        mbar_arrive(&p_full[b]);
-      }
-
-      // ---- item epilogue: O / L -> 16-bit -> swizzled staging in P buffer (g_last & 1) -> store warp
-      const int g_last = g - 1;
-      mbar_wait(&pv_done[g_last & 1], (g_last >> 1) & 1);
-      tc_fence_after_sync();
-      uint32_t o[32], lsum[16];
-      tmem_ld_32x32b_x32(tmem_base + lane_addr + TMEM_O_OFF + grp * 32, o);
-      tmem_ld_32x32b_x16(tmem_base + lane_addr + TMEM_L_OFF, lsum);
-      tmem_ld_wait_dep(o);
-      tmem_ld_wait_dep(lsum);
-      if (nkv == 1 && it > 0) mbar_wait(stg_free, (it - 1) & 1);   // single-tile items: not waited for inside the loop
-      const float inv = 1.0f / __uint_as_float(lsum[0]);
-      uint8_t* stg = smem_p + (g_last & 1) * P_BYTES + r * 128;
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        uint4 w;
-        w.x = pack2<kBF16>(__uint_as_float(o[i * 8 + 0]) * inv, __uint_as_float(o[i * 8 + 1]) * inv);
-        w.y = pack2<kBF16>(__uint_as_float(o[i * 8 + 2]) * inv, __uint_as_float(o[i * 8 + 3]) * inv);
-        w.z = pack2<kBF16>(__uint_as_float(o[i * 8 + 4]) * inv, __uint_as_float(o[i * 8 + 5]) * inv);
-        w.w = pack2<kBF16>(__uint_as_float(o[i * 8 + 6]) * inv, __uint_as_float(o[i * 8 + 7]) * inv);
-        *reinterpret_cast<uint4*>(stg + (((grp * 4 + i) ^ rsw) << 4)) = w;
-      }
-      if (kX && grp == 1) {
-        uint32_t ox[16];
-        tmem_ld_32x32b_x16(tmem_base + lane_addr + TMEM_O_OFF + HD, ox);
-        tmem_ld_wait_dep(ox);
-#pragma unroll
-        for (int c = 0; c < 2; ++c) {
-          uint4 w;
-          w.x = pack2<kBF16>(__uint_as_float(ox[c * 8 + 0]) * inv, __uint_as_float(ox[c * 8 + 1]) * inv);
-          w.y = pack2<kBF16>(__uint_as_float(ox[c * 8 + 2]) * inv, __uint_as_float(ox[c * 8 + 3]) * inv);
-          w.z = pack2<kBF16>(__uint_as_float(ox[c * 8 + 4]) * inv, __uint_as_float(ox[c * 8 + 5]) * inv);
-          w.w = pack2<kBF16>(__uint_as_float(ox[c * 8 + 6]) * inv, __uint_as_float(ox[c * 8 + 7]) * inv);
-          *reinterpret_cast<uint4*>(smem_stgx + r * 32 + ((c ^ ((r >> 2) & 1)) << 4)) = w;
-        }
-      }
-      tc_fence_before_sync();                    // the read-out above precedes, in the tensor-core proxy, whatever our next arrivals release
-      fence_proxy_async_smem();
-      mbar_arrive(stg_full);
-    }
-  }
-
-  tc_fence_before_sync();
-  __syncthreads();
-  if (warp == 2) {
-    tc_fence_after_sync();
-    tmem_dealloc<TMEM_COLS>(tmem_base);
-  }
-}
-
 
 }  // namespace attn
 
@@ -920,31 +419,6 @@ static int attention_launch_t(const AttnMaps& m, dim3 grid, int tokens, int head
   return FVS_OK;
 }
 
-template <bool kBF16, bool kX>
-static int attention_persistent_launch_t(const AttnMaps& m, int frames, int tokens, int heads, float scale_log2e,
-                                         cudaStream_t stream) {
-  using namespace attn;
-  static bool done = false;
-  if (!done) {
-    FVS_CUDA_OK(cudaFuncSetAttribute(attention_persistent_kernel<kBF16, kX>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     PLay<kX>::BYTES));
-    done = true;
-  }
-  const long long total = (long long)((tokens + BQ - 1) / BQ) * heads * frames;
-  const long long resident = 2LL * device_sm_count();     // __launch_bounds__(384, 2): two CTAs per SM stay resident
-  dim3 grid((unsigned)(total < resident ? total : resident));
-  FVS_CUDA_OK(launch_ex(attention_persistent_kernel<kBF16, kX>, grid, dim3(kThreads), PLay<kX>::BYTES, stream, 1, /*pdl=*/true,
-                        m.q, m.kv, m.ctx, m.qx, m.kvx, m.ctxx, tokens, heads, frames, scale_log2e));
-  return FVS_OK;
-}
-
-// FVS_ATTN_PERSIST=1 selects the persistent kernel, 0 the one-CTA-per-item kernel.  Read at every launch (a getenv is
-// noise next to a launch) so that one process can A/B the two and the tests can assert that they agree bit for bit.
-static bool attention_persistent() {
-  const char* e = getenv("FVS_ATTN_PERSIST");
-  return e ? (atoi(e) != 0) : (FVS_ATTN_PERSIST_DEFAULT != 0);
-}
-
 int attention_launch(const AttnMaps& m, int frames, int tokens, int heads, float scale, int dtype, cudaStream_t stream,
                      int head_dim) {
   using namespace attn;
@@ -952,18 +426,10 @@ int attention_launch(const AttnMaps& m, int frames, int tokens, int heads, float
   dim3 grid((tokens + BQ - 1) / BQ, heads, frames);
   const bool bf = dtype == FVS_BF16, x80 = head_dim == 80;
   const int prof = prof_begin(FVS_PROF_ATTENTION, 4.0 * frames * double(heads) * tokens * double(tokens) * head_dim, stream);
-  int r;
-  if (attention_persistent()) {
-    r = x80 ? (bf ? attention_persistent_launch_t<true, true>(m, frames, tokens, heads, scale_log2e, stream)
-                  : attention_persistent_launch_t<false, true>(m, frames, tokens, heads, scale_log2e, stream))
-            : (bf ? attention_persistent_launch_t<true, false>(m, frames, tokens, heads, scale_log2e, stream)
-                  : attention_persistent_launch_t<false, false>(m, frames, tokens, heads, scale_log2e, stream));
-  } else {
-    r = x80 ? (bf ? attention_launch_t<true, true>(m, grid, tokens, heads, scale_log2e, stream)
-                  : attention_launch_t<false, true>(m, grid, tokens, heads, scale_log2e, stream))
-            : (bf ? attention_launch_t<true, false>(m, grid, tokens, heads, scale_log2e, stream)
-                  : attention_launch_t<false, false>(m, grid, tokens, heads, scale_log2e, stream));
-  }
+  const int r = x80 ? (bf ? attention_launch_t<true, true>(m, grid, tokens, heads, scale_log2e, stream)
+                          : attention_launch_t<false, true>(m, grid, tokens, heads, scale_log2e, stream))
+                    : (bf ? attention_launch_t<true, false>(m, grid, tokens, heads, scale_log2e, stream)
+                          : attention_launch_t<false, false>(m, grid, tokens, heads, scale_log2e, stream));
   if (r) return r;
   prof_end(prof, stream);
   FVS_CHECK_LAUNCH("attention_kernel");

@@ -55,17 +55,11 @@ FVS_DEVICE void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes)
                : "memory");
 }
-// FVS_MBAR_WAIT_MODE selects how a waiting thread polls (per translation unit; A/B-measured, see DESIGN.md):
-//   0  try_wait with a suspend-time hint: the hardware parks the thread (NANOSLEEP.SYNCS) until the phase completes or the
-//      hint expires — cheapest in issue slots, but the wake-up adds latency to every producer->consumer hand-off
-//   1  try_wait without a hint (implementation-defined short suspend)
-//   2  test_wait: pure spin, lowest hand-off latency, burns issue slots
-#ifndef FVS_MBAR_WAIT_MODE
-#define FVS_MBAR_WAIT_MODE 0
-#endif
+// try_wait with a suspend-time hint: the hardware parks the thread (NANOSLEEP.SYNCS) until the phase completes or the hint
+// expires.  Cheapest in issue slots; a hint-less try_wait and a test_wait spin were both slower in the tcgen05 kernels
+// (DESIGN.md §3.2).
 FVS_DEVICE bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
   uint32_t ok;
-#if FVS_MBAR_WAIT_MODE == 0
   asm volatile(
       "{\n\t"
       ".reg .pred P;\n\t"
@@ -75,27 +69,6 @@ FVS_DEVICE bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
       : "=r"(ok)
       : "r"(smem_u32(bar)), "r"(parity), "r"(0x10000u)
       : "memory");
-#elif FVS_MBAR_WAIT_MODE == 1
-  asm volatile(
-      "{\n\t"
-      ".reg .pred P;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 P, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, P;\n\t"
-      "}\n"
-      : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-#else
-  asm volatile(
-      "{\n\t"
-      ".reg .pred P;\n\t"
-      "mbarrier.test_wait.parity.shared::cta.b64 P, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, P;\n\t"
-      "}\n"
-      : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-#endif
   return ok != 0;
 }
 // Wait for the phase with the given parity to complete. Traps on (very long) timeout.
